@@ -57,7 +57,7 @@ KERNEL_BYTES = {
     'heads_kernel': 4 * (1280 + 62), 'dense_recon_tc_kernel': 4 * (62 + 3 * 68), 'dense_alpha_kernel': 4 * 62,
 }
 DENSE_BYTES_PER_FACE = 3 * 53215 * 4          # SURVEY.md section 8(d): 638,580 B written per face
-MIN_TIMED_SECONDS = 2.0                       # the K steps are repeated until the timed region is this long
+DUMP_MAX_BYTES = 64 << 20                     # --dump-outputs: above this a fixed sample of faces is written
 
 
 def load_peaks():
@@ -148,6 +148,18 @@ def dominant_roofline(kernel_ms: dict, batch: int, peaks: dict):
                     f'x {batch} faces / CUDA-event time of one launch; peaks = sustained bf16 and HBM copy of {peaks["source"]}'}
 
 
+def dump_outputs(out_dir: str, lmk) -> None:
+    """--dump-outputs: the landmarks the timed path returned in its last step, as DIR/landmarks.npy (float32), so that
+    two builds run with the same arguments can be compared output for output.  Above DUMP_MAX_BYTES a seeded sample of
+    faces (the same faces on every run) is written in their original order."""
+    a = np.ascontiguousarray(lmk.cpu().numpy() if torch.is_tensor(lmk) else lmk, np.float32)
+    n_max = DUMP_MAX_BYTES // a[:1].nbytes
+    if a.shape[0] > n_max:
+        a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], n_max, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, 'landmarks.npy'), a)
+
+
 def build_model(device: str):
     """Random-init weights of the reference architecture + seeded synthetic 3DMM (no network)."""
     from synergynet_b200 import model_building, synthetic
@@ -229,8 +241,10 @@ def run_reference(args):
         step()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()
+        lmk = step()
     el = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, lmk)
     value = args.steps * sample / el
     line = {
         'metric': METRIC, 'value': value, 'unit': 'faces/s', 'n_gpus': args.gpus, 'steps': args.steps,
@@ -522,41 +536,30 @@ def run_b200(args):
             dist.barrier()
         torch.cuda.synchronize(dev)
 
-    for i in range(max(args.warmup, 3)):
-        step(i)
-    barrier()
-    # The K steps the driver asks for are repeated `rounds` times inside ONE timed region so that it lasts
-    # >= MIN_TIMED_SECONDS (sustained clocks, >= 10 clock samples); ms_per_step = region / (rounds * K).
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
-    for i in range(args.steps):
-        step(i)
-    if world > 1:
-        og.wait()
-    e1.record()
-    barrier()
-    probe_ms = max(e0.elapsed_time(e1), 1e-3)
-    rounds = 1 if args.profile else max(1, int(np.ceil(MIN_TIMED_SECONDS * 1e3 / probe_ms)))
-    r = torch.tensor([rounds], device=dev, dtype=torch.int64)
-    if world > 1:
-        dist.all_reduce(r, op=dist.ReduceOp.MAX)
-    rounds = int(r.item())
     sampler = ClockSampler(local_rank) if rank == 0 else None
     if sampler:
         sampler.start()
-        time.sleep(0.25)
+        t_start = time.time()
+        while sampler.proc is not None and not sampler.rows and time.time() - t_start < 5.0:
+            time.sleep(0.01)                            # nvidia-smi's start-up stays out of the timed steps
+    # the warm-up runs after the sampler's start-up, right before the timed steps, so that they do not begin on an idle
+    # GPU whose clocks have dropped
+    for i in range(max(args.warmup, 3)):
+        step(i)
+    barrier()
     launches0 = eng.launch_count
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    barrier()
     t_wall0 = time.time()
     ev0.record()
-    for i in range(rounds * args.steps):
-        step(i)
+    for i in range(args.steps):
+        lmk = step(i)
     if world > 1:
         og.wait()                                       # the last gather ends inside the CUDA-event region
     ev1.record()
     barrier()
     t_wall1 = time.time()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, lmk_alls[(args.steps - 1) & 1] if world > 1 else lmk)
     ms = ev0.elapsed_time(ev1)
     launches = eng.launch_count - launches0
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
@@ -564,7 +567,7 @@ def run_b200(args):
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms = float(t.item())
-    n_timed = rounds * args.steps
+    n_timed = args.steps
     eng.raise_if_error()
 
     # ---- multi-GPU correctness: the gathered tensor holds every rank's shard in rank order -----------------
@@ -742,8 +745,8 @@ def run_b200(args):
                        'collective': ('one all_gather_into_tensor of the (B,3,68) landmarks per step (NCCL), issued on a side '
                                       'stream under the next step\'s backbone; the last one completes inside the timed region'
                                       if world > 1 else None),
-                       'timed_region': f'{rounds} x {args.steps} steps in one CUDA-event region ({ms / 1e3:.2f} s)',
-                       'rounds': rounds, 'timed_steps': n_timed,
+                       'timed_region': f'{args.steps} steps in one CUDA-event region ({ms / 1e3:.2f} s)',
+                       'timed_steps': n_timed,
                        'l2': f'{n_rot} rotating device-resident input batches of {B * X_BYTES_PER_FACE / 1e6:.0f} MB '
                              '(> 126 MB L2) + >1 GB of activations written per step'},
             'e2e': {'value': world * B * e2e_steps / e2e_s, 'unit': 'faces/s',
@@ -810,7 +813,11 @@ def main():
     ap.add_argument('--no-config5', action='store_true', help='skip the ResNet-50 / PointNet heads measurement')
     ap.add_argument('--no-render', action='store_true', help='skip the Sim3DR / FaceBoxes post-processing measurement')
     ap.add_argument('--no-single-pass', action='store_true', help='skip the single-pass fp16 engine measurement')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the landmarks of the last timed step to DIR/landmarks.npy (float32, at most 64 MB)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         run_reference(args)
     else:

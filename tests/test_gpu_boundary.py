@@ -12,6 +12,7 @@ import pytest
 import torch
 import torch.nn as nn
 
+from oracle import golden
 from oracle import reference_port as rp
 from oracle import synth_model
 from synergynet_b200 import _lib, synthetic
@@ -113,7 +114,7 @@ def test_cpu_constructed_wrapper_runs_like_the_reference(synth_pack, sd, basis):
     lmk = model.reconstruct_vertex_62(params)
     assert not lmk.is_cuda
     assert rp.max_rel_err(lmk.numpy(), rp.reconstruct_vertex_62(want.numpy(), basis)) < TOL
-    gold = dict(np.load(__import__('os').path.join(__import__('os').path.dirname(__file__), 'golden', 'ref_vectors.npz')))
+    gold = golden.load_ref_vectors()
     rects = [list(r) for r in gold['scene_rects']]
     pts, verts, poses = model.get_all_outputs(gold['scene'].copy(), rects=rects)
     assert rp.max_rel_err(np.stack(pts), gold['scene_lmk']) < TOL

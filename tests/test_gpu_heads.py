@@ -1,18 +1,17 @@
 """SURVEY.md section 8 rows a10 / f4 on the B200: MLP_for / MLP_rev, WingLoss / ParamLoss and SynergyNet.forward
 (inference mode) through the C ABI, against the vectors recorded from the reference's own modules and the CPU oracle."""
-import os
 import types
 
 import numpy as np
 import pytest
 import torch
 
+from oracle import golden
 from oracle import reference_port as rp
 from oracle import synth_model
 from synergynet_b200 import synthetic
 
 pytestmark = pytest.mark.gpu
-GOLD = os.path.join(os.path.dirname(__file__), 'golden', 'ref_vectors.npz')
 TOL = 1e-4
 # The PointNet heads are nine random, BatchNorm-calibrated layers in a row: they amplify a relative perturbation of their
 # input ~50x (measured on the oracle: 1e-6 on the landmarks -> 4.8e-5 on point_residual), and the reference's own fp32 result
@@ -25,7 +24,7 @@ LOSS_KEYS = ('loss_LMK_f0', 'loss_LMK_pointNet', 'loss_Param_In', 'loss_Param_S2
 
 @pytest.fixture(scope='module')
 def gold():
-    return dict(np.load(GOLD, allow_pickle=False))
+    return golden.load_ref_vectors()
 
 
 @pytest.fixture(scope='module')

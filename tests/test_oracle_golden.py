@@ -1,22 +1,21 @@
 """Pin the CPU oracle (oracle/reference_port.py) to the vectors recorded from the live reference
 (tests/golden/make_golden.py).  CPU only."""
-import os
 
 import numpy as np
 import pytest
 import torch
 
+from oracle import golden
 from oracle import reference_port as rp
 from oracle import synth_model
 from synergynet_b200 import synthetic
 
-GOLD = os.path.join(os.path.dirname(__file__), 'golden', 'ref_vectors.npz')
 TOL = 2e-5       # oracle and reference run the same ATen kernels; slack is for cross-host ISA paths
 
 
 @pytest.fixture(scope='module')
 def gold():
-    return dict(np.load(GOLD, allow_pickle=False))
+    return golden.load_ref_vectors()
 
 
 @pytest.fixture(scope='module')
@@ -124,4 +123,8 @@ def test_thousand_face_batch_sample(gold, sd, basis):
     idx = torch.arange(0, 1024, 64)
     p, _ = rp.mobilenetv2_forward(sd, xs[idx])
     assert rp.max_rel_err(p.numpy(), gold['params1024'][idx.numpy()]) < TOL
-    assert rp.max_rel_err(rp.reconstruct_vertex_62(p.numpy(), basis), gold['lmk1024'][idx.numpy()]) < TOL
+    assert rp.max_rel_err(rp.reconstruct_vertex_62(p.numpy(), basis), gold['lmk1024_even'][idx.numpy() // 2]) < TOL
+    # the reconstruction of the reference's own parameters, which stands in for the landmarks not stored (odd faces)
+    lmk = rp.reconstruct_vertex_62(gold['params1024'][::2], basis)
+    assert rp.max_rel_err(lmk, gold['lmk1024_even']) < 1e-6
+    assert rp.nme_vs_reference(lmk, gold['lmk1024_even']).max() < 1e-6

@@ -1,11 +1,12 @@
 """Pin the render / detection oracle (oracle/render_port.py, oracle/sim3dr_port.c) to the vectors recorded from the live
-reference (tests/golden/make_golden_render.py) and, where it has been built, to the reference's own C++ compiled in place
-(oracle/_ref/libsim3dr_ref.so).  CPU only."""
+reference (tests/golden/make_golden_render.py) and from the reference's own C++ compiled unmodified
+(tests/golden/make_golden_sim3dr.py).  CPU only."""
 import os
 
 import numpy as np
 import pytest
 
+from oracle import golden
 from oracle import render_port as rp
 from synergynet_b200 import synthetic
 
@@ -54,24 +55,19 @@ def test_pipeline_sequence(gold):
         assert np.array_equal(img, gold['render_steps'][b])
 
 
-@pytest.mark.skipif(not rp.have_ref(), reason='oracle/_ref not built (no /root/reference on this host)')
 def test_port_equals_compiled_reference():
-    tri = synthetic.make_render_topology(60, 70)
-    verts = synthetic.make_render_meshes(2, 200, 240, seed=5, rows=60, cols=70, size=120)
-    rng = np.random.default_rng(3)
-    # a few huge and degenerate triangles on top of the mesh
-    extra = np.array([[0, 4199, 2100], [10, 10, 500], [69, 4130, 35]], np.int32)
-    tri = np.ascontiguousarray(np.concatenate([tri, extra]))
+    """Bit for bit against the reference's own rasterize_kernel.cpp (tests/golden/make_golden_sim3dr.py), on meshes with
+    a few huge and degenerate triangles on top of the grid."""
+    ref = golden.load_sim3dr_ref_vectors()
+    tri = ref['tri']
     for b in range(2):
-        ver = np.ascontiguousarray(verts[b].T)
-        n_p, n_r = rp.get_normal(ver, tri, 'port'), rp.get_normal(ver, tri, 'ref')
-        assert np.array_equal(n_p, n_r, equal_nan=True)
-        col = rng.uniform(0, 1, ver.shape).astype(np.float32)
-        bg = rng.integers(0, 256, (200, 240, 3), dtype=np.uint8)
+        ver = np.ascontiguousarray(ref['verts'][b].T)
+        assert np.array_equal(rp.get_normal(ver, tri, 'port'), ref['normals'][b], equal_nan=True)
+        bg = ref['bg'][b]
         for rev in (False, True):
-            a, da = rp.rasterize(ver, tri, col, bg.copy(), reverse=rev, kind='port', return_depth=True)
-            r, dr = rp.rasterize(ver, tri, col, bg.copy(), reverse=rev, kind='ref', return_depth=True)
-            assert np.array_equal(a, r) and np.array_equal(da, dr)
+            a, da = rp.rasterize(ver, tri, ref['colors'][b], bg.copy(), reverse=rev, kind='port', return_depth=True)
+            assert np.array_equal(a - bg, ref['image_minus_bg'][b, int(rev)]) and np.array_equal(da, ref['depth'][b, int(rev)])
+    assert ref['image_minus_bg'].any()
 
 
 def test_prior_boxes_bit_exact(gold):
