@@ -196,6 +196,36 @@ int syn_resnet_commit(syn_handle_t* h);                      /* after syn_commit
 int syn_resnet50_forward(syn_handle_t* h, const float* x_dev, int batch, float* out102_dev, float* pool2048_dev,
                          void* stream);
 
+/* ---- ResNeSt-50 backbone variant (model_building.py:48-49, I2P with any arch containing 'resnest';
+ * backbone_nets/ResNeSt/resnest.py:33-41, resnet.py:29-324, splat.py:11-98) -------------------------------------------
+ * 87 parameterised layers in execution order: the deep stem conv1.0, conv1.3, conv1.6 (resnet.py:182-190; conv1.6 is
+ * followed by the top-level bn1, :299-300); then per Bottleneck conv1, conv2.conv (3x3, groups 2), conv2.fc1,
+ * conv2.fc2, conv3 and -- first block of a stage -- downsample.1, the 1x1 conv behind the avg-down pool (:246-261).
+ * syn_resnest_layer_desc names each with the checkpoint's own key prefixes: name = the conv ("<name>.weight",
+ * "<name>.bias" when has_bias), bn_name = its eval-mode BatchNorm2d ("<bn_name>.weight/.bias/.running_mean/
+ * .running_var") or NULL for conv2.fc2, the one layer without one (splat.py:42).  h_in / h_out are the spatial sizes
+ * the layer runs at (conv2 runs at stride 1: the avd AvgPool2d(3, 2, 1) after it downsamples, resnet.py:45-50).
+ * syn_resnest_set_layer: w_host OIHW fp32 of cout * cin/groups * ksize^2 values (else SYN_ERR_SHAPE); bias_host and
+ * the four BatchNorm tensors must be given exactly when the layer has them (else SYN_ERR_INVALID).
+ * Heads: fc_ori | fc_shape | fc_exp concatenated in the reference's output order -> (62, 2048), (62) (resnet.py:316-320;
+ * fc_tex is in the checkpoint but never evaluated, :319).
+ * syn_resnest50_forward: x_dev (B,3,120,120) NCHW -> out62_dev (B,62) and pool2048_dev (B,2048) (may be NULL), the
+ * (x, avgpool) pair ResNet.forward returns (:298-324).  SYN_ERR_STATE before syn_resnest_commit. */
+typedef struct {
+  const char* name;
+  const char* bn_name;
+  int32_t cin, cout, ksize, stride, groups, has_bias, h_in, h_out;
+} syn_resnest_layer_desc_t;
+int syn_resnest_num_layers(void);                            /* 87 */
+int syn_resnest_layer_desc(int idx, syn_resnest_layer_desc_t* out);
+int syn_resnest_set_layer(syn_handle_t* h, int idx, const float* w_host, int64_t w_numel, const float* bias_host,
+                          const float* bn_weight_host, const float* bn_bias_host, const float* bn_mean_host,
+                          const float* bn_var_host, float eps);
+int syn_resnest_set_heads(syn_handle_t* h, const float* w62x2048_host, const float* b62_host);
+int syn_resnest_commit(syn_handle_t* h);                     /* after syn_commit */
+int syn_resnest50_forward(syn_handle_t* h, const float* x_dev, int batch, float* out62_dev, float* pool2048_dev,
+                          void* stream);
+
 /* ---- Sim3DR: vertex normals, lighting, z-buffer rasterisation (SURVEY.md section 8 row f2) -------------------------
  * Handle-free; every pointer is caller-owned device memory unless it says _host.  B meshes share one triangle list
  * tri_dev (ntri,3) int32, 0-based (utils/render.py:32-33).  Vertices are read in place through element strides:

@@ -7,7 +7,7 @@ import types
 import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from oracle import synth_model  # noqa: E402
+from oracle import resnest_port, synth_model  # noqa: E402
 from synergynet_b200 import inference, model_building, synthetic  # noqa: E402
 from synergynet_b200.params import ParamsPack, set_param_pack  # noqa: E402
 
@@ -44,6 +44,11 @@ def main():
     rn.load_state_dict({'I2P.backbone.' + k: v for k, v in synth_model.build_resnet50_state_dict(0).items()}, strict=False)
     rn.eval()
     rn.forward_test(x[:2])
+    torch.cuda.synchronize()
+    rs = model_building.SynergyNet(types.SimpleNamespace(arch='resnest50', img_size=120, devices_id=[0]))
+    rs.load_state_dict({'I2P.backbone.' + k: v for k, v in resnest_port.build_resnest50_state_dict(0).items()}, strict=False)
+    rs.eval()
+    rs.forward_test(x[:2])
     torch.cuda.synchronize()
     eng.raise_if_error()
     print('sanitizer smoke done:', float(dense.abs().max()), {k: float(v.mean()) for k, v in loss.items()})

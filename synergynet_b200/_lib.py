@@ -42,6 +42,12 @@ class FbLayerDesc(C.Structure):
     _fields_ = [('name', C.c_char_p)] + [(n, C.c_int32) for n in ('cin', 'cout', 'ksize', 'stride', 'pad', 'has_bn', 'activation')]
 
 
+class ResNeStLayerDesc(C.Structure):
+    """``syn_resnest_layer_desc_t``."""
+    _fields_ = [('name', C.c_char_p), ('bn_name', C.c_char_p)] + [
+        (n, C.c_int32) for n in ('cin', 'cout', 'ksize', 'stride', 'groups', 'has_bias', 'h_in', 'h_out')]
+
+
 NMS_CPU_NMS, NMS_PY_CPU_NMS = 0, 1
 
 _P, _F, _I, _L = C.c_void_p, C.c_void_p, C.c_int, C.c_int64
@@ -84,6 +90,12 @@ SIGNATURES = {
     'syn_resnet_set_heads': (_I, [_P, _F, _F]),
     'syn_resnet_commit': (_I, [_P]),
     'syn_resnet50_forward': (_I, [_P, _F, _I, _F, _F, _P]),
+    'syn_resnest_num_layers': (_I, []),
+    'syn_resnest_layer_desc': (_I, [_I, C.POINTER(ResNeStLayerDesc)]),
+    'syn_resnest_set_layer': (_I, [_P, _I, _F, _L, _F, _F, _F, _F, _F, C.c_float]),
+    'syn_resnest_set_heads': (_I, [_P, _F, _F]),
+    'syn_resnest_commit': (_I, [_P]),
+    'syn_resnest50_forward': (_I, [_P, _F, _I, _F, _F, _P]),
     'syn_debug_heads_buffer': (_I, [_P, _I, _F, _L]),
     'syn_mesh_incidence_host': (_I, [_F, _I, _I, _F, _F]),
     'syn_mesh_normals': (_I, [_F, _L, _I, _I, _I, _I, _F, _I, _F, _F, _F, _F, _P]),
@@ -116,6 +128,8 @@ _CORE = {n for n in SIGNATURES if n not in ('syn_peek_error', 'syn_poll_saturati
                                              'syn_pointnet_commit', 'syn_mlp_for', 'syn_mlp_rev', 'syn_wing_loss',
                                              'syn_param_loss', 'syn_reconstruct_image', 'syn_pose_decode', 'syn_set_center_crop', 'syn_resnet_num_convs', 'syn_resnet_conv_desc',
                                              'syn_resnet_set_conv', 'syn_resnet_set_heads', 'syn_resnet_commit', 'syn_resnet50_forward', 'syn_debug_heads_buffer',
+                                             'syn_resnest_num_layers', 'syn_resnest_layer_desc', 'syn_resnest_set_layer',
+                                             'syn_resnest_set_heads', 'syn_resnest_commit', 'syn_resnest50_forward',
                                              'syn_mesh_incidence_host', 'syn_mesh_normals', 'syn_mesh_lighting', 'syn_rasterize', 'syn_nms',
                                              'syn_faceboxes_num_priors', 'syn_faceboxes_decode', 'syn_fb_num_layers', 'syn_fb_layer_desc', 'syn_fb_create',
                                              'syn_fb_destroy', 'syn_fb_set_layer', 'syn_fb_commit', 'syn_fb_forward', 'syn_fb_launch_count')}

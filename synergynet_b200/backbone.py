@@ -258,3 +258,89 @@ def resnet50_conv_keys():
 
 def resnet50(pretrained: bool = False, **_):
     return ResNet50Params()
+
+
+# ---- ResNeSt-50 backbone variant (reference backbone_nets/ResNeSt/resnest.py:33-41, resnet.py:29-324, splat.py) ------
+
+class _SplAtParams(nn.Module):
+    """``SplAtConv2d`` with radix 2, cardinality 1 (splat.py:14-45): conv (groups 2), bn0, fc1 (+bias), bn1, fc2 (+bias)."""
+
+    def __init__(self, gw):
+        super().__init__()
+        inter = max(gw * 2 // 4, 32)
+        self.conv = nn.Conv2d(gw, gw * 2, 3, 1, 1, groups=2, bias=False)
+        self.bn0 = nn.BatchNorm2d(gw * 2)
+        self.fc1 = nn.Conv2d(gw, inter, 1)
+        self.bn1 = nn.BatchNorm2d(inter)
+        self.fc2 = nn.Conv2d(inter, gw * 2, 1)
+
+
+class _SplAtBottleneck(nn.Module):
+    expansion = 4
+
+    def __init__(self, inplanes, planes, downsample=None):
+        super().__init__()
+        self.conv1 = nn.Conv2d(inplanes, planes, 1, bias=False)
+        self.bn1 = nn.BatchNorm2d(planes)
+        self.conv2 = _SplAtParams(planes)
+        self.conv3 = nn.Conv2d(planes, planes * 4, 1, bias=False)
+        self.bn3 = nn.BatchNorm2d(planes * 4)
+        self.downsample = downsample
+
+
+RESNEST_STAGES = ((64, 3, 1), (128, 4, 2), (256, 6, 2), (512, 3, 2))     # (planes, blocks, stride), resnet.py:197-219
+
+
+class ResNeSt50Params(nn.Module):
+    """Key schema of ``ResNeSt.resnest50()`` (482 state-dict keys): the deep stem ``conv1.{0,1,3,4,6}`` + ``bn1``,
+    ``layer1..4.{i}.conv1/bn1/conv2.{conv,bn0,fc1,bn1,fc2}/conv3/bn3/downsample.{1,2}``, fc_ori/fc_shape/fc_exp/fc_tex.
+    Parameter container; the forward pass runs in the sm_100a library."""
+    feature_dim = 2048
+
+    def __init__(self):
+        super().__init__()
+        self.conv1 = nn.Sequential(nn.Conv2d(3, 32, 3, 2, 1, bias=False), nn.BatchNorm2d(32), nn.ReLU(inplace=True),
+                                   nn.Conv2d(32, 32, 3, 1, 1, bias=False), nn.BatchNorm2d(32), nn.ReLU(inplace=True),
+                                   nn.Conv2d(32, 64, 3, 1, 1, bias=False))
+        self.bn1 = nn.BatchNorm2d(64)
+        inplanes = 64
+        for li, (planes, blocks, stride) in enumerate(RESNEST_STAGES, 1):
+            layers = []
+            for j in range(blocks):
+                ds = None
+                if j == 0:          # avg-down shortcut: AvgPool2d (identity in layer1), 1x1 conv, BN (resnet.py:246-261)
+                    ds = nn.Sequential(nn.AvgPool2d(stride, stride, ceil_mode=True, count_include_pad=False),
+                                       nn.Conv2d(inplanes, planes * 4, 1, bias=False), nn.BatchNorm2d(planes * 4))
+                layers.append(_SplAtBottleneck(inplanes, planes, ds))
+                inplanes = planes * 4
+            setattr(self, f'layer{li}', nn.Sequential(*layers))
+        self.fc_ori = nn.Linear(2048, 12)
+        self.fc_shape = nn.Linear(2048, 40)
+        self.fc_exp = nn.Linear(2048, 10)
+        self.fc_tex = nn.Linear(2048, 40)
+        for m in self.modules():                                            # resnet.py:235-241
+            if isinstance(m, nn.Conv2d):
+                m.weight.data.normal_(0, (2.0 / (m.kernel_size[0] * m.kernel_size[1] * m.out_channels)) ** 0.5)
+            elif isinstance(m, nn.BatchNorm2d):
+                m.weight.data.fill_(1)
+                m.bias.data.zero_()
+
+    def forward(self, *a, **k):  # pragma: no cover
+        raise RuntimeError('ResNeSt50Params is a parameter container; the forward pass runs in the sm_100a library')
+
+
+def resnest50_layer_keys():
+    """(conv key, BatchNorm key or None) of the 87 layers in the execution order of the C ABI (syn_resnest_set_layer)."""
+    keys = [('conv1.0', 'conv1.1'), ('conv1.3', 'conv1.4'), ('conv1.6', 'bn1')]
+    for li, (_, blocks, _) in enumerate(RESNEST_STAGES, 1):
+        for j in range(blocks):
+            pre = f'layer{li}.{j}'
+            keys += [(f'{pre}.conv1', f'{pre}.bn1'), (f'{pre}.conv2.conv', f'{pre}.conv2.bn0'),
+                     (f'{pre}.conv2.fc1', f'{pre}.conv2.bn1'), (f'{pre}.conv2.fc2', None), (f'{pre}.conv3', f'{pre}.bn3')]
+            if j == 0:
+                keys.append((f'{pre}.downsample.1', f'{pre}.downsample.2'))
+    return keys
+
+
+def resnest50(pretrained: bool = False, **_):
+    return ResNeSt50Params()

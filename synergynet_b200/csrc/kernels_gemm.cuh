@@ -1,7 +1,8 @@
 // General fp32-accurate GEMM / implicit-GEMM convolution on tcgen05 for the layers outside the fused MobileNetV2
 // blocks: the PointNet refinement heads MLP_for / MLP_rev (reference backbone_nets/pointnet_backbone.py:31-64,
-// 90-106; Conv1d(k=1) + BatchNorm1d + ReLU over B x 68 points) and the ResNet-50 backbone variant
-// (backbone_nets/resnet_backbone.py:227-249; 1x1 / 3x3 convolutions + BatchNorm2d + ReLU, NHWC here).
+// 90-106; Conv1d(k=1) + BatchNorm1d + ReLU over B x 68 points), the ResNet-50 backbone variant
+// (backbone_nets/resnet_backbone.py:227-249; 1x1 / 3x3 convolutions + BatchNorm2d + ReLU, NHWC here) and the
+// ResNeSt-50 variant (backbone_nets/ResNeSt/resnet.py, splat.py; including the radix-2 grouped 3x3 convolution).
 //
 //   out[m, n] = act( sum_k A[m, k] * W[n, k] * oscale[n] + bias[n] + addend[m / group, n] + residual[m, n] )
 //
@@ -49,6 +50,15 @@ struct GemmArgs {
   int M, K, N, Kp, nr, lda, act;
   // conv mode (ksize > 0): implicit GEMM over k = (ky * ksize + kx) * C + c
   int ksize, stride, pad, H, W, C, HO, WO;
+  // grouped conv mode: C is the per-group input channel count, a_pix the channel count of an input pixel (= C when
+  // ungrouped); the CTA of n-range n0 is in group n0 / n_group (n_group = output channels per group, 0 = ungrouped;
+  // nr divides it) and reads input channels [group * C, (group + 1) * C)
+  int n_group, a_pix;
+  // accumulator split (0 = one TMEM accumulator for all three passes).  The tensor cores round each accumulator update
+  // toward zero, so the error of a sum grows with the number of updates times the accumulator's magnitude; with
+  // acc_slices = S > 0 the hi*hi products of chunk c go to accumulator c % S and the two small correction passes to a
+  // separate one (S + 1 buffers of nr columns in a 512-column allocation), summed in fp32 by the epilogue
+  int acc_slices;
   int* err;
 };
 
@@ -75,6 +85,7 @@ __global__ void __launch_bounds__(kGmThreads, 1) tc_gemm_kernel(const GemmArgs p
     s_osc[i] = p.oscale[n0 + i];
   }
   const int nchunks = (p.Kp + kGmKC - 1) / kGmKC;
+  const int nsl = min(p.acc_slices, nchunks);                  // hi*hi slices in use (split accumulators), 0 = off
   const uint8_t* wimg = p.Wimg + (size_t)blockIdx.y * (size_t)p.nr * p.Kp * 4;
 
   if (tid == 0) {
@@ -85,7 +96,10 @@ __global__ void __launch_bounds__(kGmThreads, 1) tc_gemm_kernel(const GemmArgs p
     mbar_init(smem_u32(&bar_acc), 1);
     fence_mbar_init();
   }
-  if (warp == kGmProducerWarps) tmem_alloc<256>(smem_u32(&tmem_base_s));
+  if (warp == kGmProducerWarps) {
+    if (p.acc_slices > 0) tmem_alloc<512>(smem_u32(&tmem_base_s));
+    else tmem_alloc<256>(smem_u32(&tmem_base_s));
+  }
   tc_fence_before_sync();
   __syncthreads();
   tc_fence_after_sync();
@@ -116,6 +130,7 @@ __global__ void __launch_bounds__(kGmThreads, 1) tc_gemm_kernel(const GemmArgs p
     const int e_row = gemm_row_exp(mx);
     const float a_scale = exp2i(e_row);
     const float* arow = p.A + (size_t)m * p.lda;
+    const float* abase = p.A + (p.n_group > 0 ? (n0 / p.n_group) * p.C : 0);   // grouped conv: this CTA's input channels
     for (int c = 0; c < nchunks; ++c) {
       const int s = c % kGmStages, use = c / kGmStages;
       const int k0 = c * kGmKC;
@@ -131,7 +146,7 @@ __global__ void __launch_bounds__(kGmThreads, 1) tc_gemm_kernel(const GemmArgs p
             const int tap = k / p.C, cc = k - tap * p.C;
             const int ky = tap / p.ksize, kx = tap - ky * p.ksize;
             const int iy = oy * p.stride - p.pad + ky, ix = ox * p.stride - p.pad + kx;
-            if (iy >= 0 && iy < p.H && ix >= 0 && ix < p.W) src = p.A + (((size_t)b * p.H + iy) * p.W + ix) * p.C + cc;
+            if (iy >= 0 && iy < p.H && ix >= 0 && ix < p.W) src = abase + (((size_t)b * p.H + iy) * p.W + ix) * p.a_pix + cc;
           } else {
             src = arow + k;
           }
@@ -189,6 +204,12 @@ __global__ void __launch_bounds__(kGmThreads, 1) tc_gemm_kernel(const GemmArgs p
     for (int c0 = kh * 16; c0 < ncols; c0 += 32) {          // the two warps of a lane quarter interleave 16-column blocks
       float v[16];
       tmem_ld16(trow + c0, v);                              // warp-collective: the control flow below stays warp-uniform
+      for (int sl = 1; sl <= nsl; ++sl) {                   // split accumulators: the other hi*hi slices, the corrections
+        float u[16];
+        tmem_ld16(trow + sl * p.nr + c0, u);
+#pragma unroll
+        for (int j = 0; j < 16; ++j) v[j] += u[j];
+      }
       if (vec && c0 + 16 <= ncols) {
 #pragma unroll
         for (int j = 0; j < 16; j += 4) {
@@ -255,9 +276,15 @@ __global__ void __launch_bounds__(kGmThreads, 1) tc_gemm_kernel(const GemmArgs p
 #pragma unroll
         for (int pass = 0; pass < 3; ++pass) {                 // hi*hi, hi*lo, lo*hi
           const uint32_t a_off = (pass == 2 ? kGmStageA : 0), b_off = (pass == 1 ? kGmStageB : 0);
+          uint32_t d = tmem, acc = (c > 0 || pass > 0) ? 1u : 0u;
+          if (nsl > 0) {                                       // split accumulators (see GemmArgs::acc_slices)
+            const int sl = pass == 0 ? c % nsl : nsl;
+            d = tmem + (uint32_t)(sl * p.nr);
+            acc = (pass == 0 ? c >= nsl : (c > 0 || pass > 1)) ? 1u : 0u;
+          }
           for (int ks = 0; ks < kc / 16; ++ks)
-            umma_f16(tmem, desc64(d_hi, a_lo + ((a_off + ks * 4096) >> 4)), desc64(d_hi, b_lo + ((b_off + ks * 2 * lbo_b) >> 4)),
-                     idesc, (c > 0 || pass > 0 || ks > 0) ? 1u : 0u);
+            umma_f16(d, desc64(d_hi, a_lo + ((a_off + ks * 4096) >> 4)), desc64(d_hi, b_lo + ((b_off + ks * 2 * lbo_b) >> 4)),
+                     idesc, (acc || ks > 0) ? 1u : 0u);
         }
         umma_commit(smem_u32(&bar_empty[s]));
         if (c == nchunks - 1) umma_commit(smem_u32(&bar_acc));
@@ -275,7 +302,8 @@ __global__ void __launch_bounds__(kGmThreads, 1) tc_gemm_kernel(const GemmArgs p
   __syncthreads();
   if (warp == kGmProducerWarps) {
     __syncwarp();
-    tmem_dealloc<256>(tmem);
+    if (p.acc_slices > 0) tmem_dealloc<512>(tmem);
+    else tmem_dealloc<256>(tmem);
   }
 }
 

@@ -81,15 +81,20 @@ __global__ void pose_decode_kernel(const float* __restrict__ params, const float
 }
 
 // -------------------------------------------------------------------------------------------------
-// Stem: (B,3,120,120) NCHW -> (B,60,60,32) NHWC, 3x3 stride 2 pad 1, +bias, ReLU6.
+// Stem: (B,3,120,120) NCHW -> (B,60,60,32) NHWC, 3x3 stride 2 pad 1, +bias, then
+//   kRelu6 = true:  ReLU6                       (MobileNetV2 features.0, mobilenetv2_backbone.py:127)
+//   kRelu6 = false: ReLU, and max|y| per output pixel into rowmax (ResNeSt-50 deep stem conv1.0-2,
+//                   ResNeSt/resnet.py:182-185; the next layer is a dynamically scaled tc_gemm conv)
 // One CTA per output row (b, oy); 256 threads = 64 pixel slots x 4 channel groups of 8.
 // Weights packed [27][32] with tap index (ci*3+ky)*3+kx.
 // -------------------------------------------------------------------------------------------------
 constexpr int kStemThreads = 256;
 
+template <bool kRelu6>
 __global__ void __launch_bounds__(kStemThreads)
 stem_conv3x3s2_kernel(const float* __restrict__ x, const float* __restrict__ w,
-                      const float* __restrict__ bias, float* __restrict__ y, int batch) {
+                      const float* __restrict__ bias, float* __restrict__ y, int batch,
+                      unsigned* __restrict__ rowmax) {
   constexpr int HI = kImg, HO = 60, CO = 32;
   __shared__ float s_in[3][3][HI + 4];   // [ci][ky][ix+1], column 0 is the left zero pad
   __shared__ __align__(16) float s_w[27 * CO];
@@ -108,7 +113,9 @@ stem_conv3x3s2_kernel(const float* __restrict__ x, const float* __restrict__ w,
   }
   __syncthreads();
   const int px = tid >> 2, cg = tid & 3;
-  if (px >= HO) return;
+  if (kRelu6 && px >= HO) return;
+  // rowmax variant: the idle slots (px >= HO) stay for the shuffles of the pixel maximum and compute a valid pixel
+  const int pxc = px < HO ? px : HO - 1;
   float acc[8];
 #pragma unroll
   for (int j = 0; j < 8; ++j) acc[j] = s_b[cg * 8 + j];
@@ -118,7 +125,7 @@ stem_conv3x3s2_kernel(const float* __restrict__ x, const float* __restrict__ w,
     for (int ky = 0; ky < 3; ++ky)
 #pragma unroll
       for (int kx = 0; kx < 3; ++kx) {
-        const float v = s_in[ci][ky][2 * px + kx];
+        const float v = s_in[ci][ky][2 * pxc + kx];
         const float4 w0 = *reinterpret_cast<const float4*>(&s_w[((ci * 3 + ky) * 3 + kx) * CO + cg * 8]);
         const float4 w1 = *reinterpret_cast<const float4*>(&s_w[((ci * 3 + ky) * 3 + kx) * CO + cg * 8 + 4]);
         acc[0] = fmaf(v, w0.x, acc[0]); acc[1] = fmaf(v, w0.y, acc[1]);
@@ -126,9 +133,25 @@ stem_conv3x3s2_kernel(const float* __restrict__ x, const float* __restrict__ w,
         acc[4] = fmaf(v, w1.x, acc[4]); acc[5] = fmaf(v, w1.y, acc[5]);
         acc[6] = fmaf(v, w1.z, acc[6]); acc[7] = fmaf(v, w1.w, acc[7]);
       }
-  float4* out = reinterpret_cast<float4*>(y + ((size_t)(b * HO + oy) * HO + px) * CO + cg * 8);
-  out[0] = make_float4(relu6f(acc[0]), relu6f(acc[1]), relu6f(acc[2]), relu6f(acc[3]));
-  out[1] = make_float4(relu6f(acc[4]), relu6f(acc[5]), relu6f(acc[6]), relu6f(acc[7]));
+  float4* out = reinterpret_cast<float4*>(y + ((size_t)(b * HO + oy) * HO + pxc) * CO + cg * 8);
+  if (kRelu6) {
+    out[0] = make_float4(relu6f(acc[0]), relu6f(acc[1]), relu6f(acc[2]), relu6f(acc[3]));
+    out[1] = make_float4(relu6f(acc[4]), relu6f(acc[5]), relu6f(acc[6]), relu6f(acc[7]));
+  } else {
+    float m = 0.f;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      acc[j] = fmaxf(acc[j], 0.f);
+      m = fmaxf(m, acc[j]);
+    }
+    if (px < HO) {
+      out[0] = make_float4(acc[0], acc[1], acc[2], acc[3]);
+      out[1] = make_float4(acc[4], acc[5], acc[6], acc[7]);
+    }
+    m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, 1));      // the 4 channel groups of a pixel are adjacent lanes
+    m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, 2));
+    if (px < HO && cg == 0) rowmax[((size_t)b * HO + oy) * HO + px] = __float_as_uint(m);
+  }
 }
 
 // -------------------------------------------------------------------------------------------------

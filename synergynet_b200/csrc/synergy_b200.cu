@@ -6,6 +6,7 @@
 
 #include <algorithm>
 #include <new>
+#include <string>
 #include <vector>
 
 #include "common.cuh"
@@ -17,6 +18,7 @@
 #include "kernels_gemm.cuh"
 #include "kernels_loss.cuh"
 #include "kernels_resnet.cuh"
+#include "kernels_resnest.cuh"
 
 using namespace syn;
 
@@ -39,11 +41,14 @@ struct syn_heads;       // PointNet refinement heads (heads_host.inl)
 void syn_heads_destroy(syn_heads* s);
 struct syn_resnet;      // ResNet-50 backbone variant (resnet_host.inl)
 void syn_resnet_destroy(syn_resnet* s);
+struct syn_resnest;     // ResNeSt-50 backbone variant (resnest_host.inl)
+void syn_resnest_destroy(syn_resnest* s);
 
 struct syn_handle {
   int device = 0;
   syn_heads* heads = nullptr;
   syn_resnet* resnet = nullptr;
+  syn_resnest* resnest = nullptr;
   int sm_count = 0;
   int engine = SYN_ENGINE_TC_FUSED;            // default: fused tcgen05 engine; 0/1 remain for cross-checks
   int center_crop = 0;                         // CenterCrop margin applied by the uint8 entry points (syn_set_center_crop)
@@ -302,8 +307,8 @@ int run_backbone(syn_handle* h, const float* x, int batch, float* params, float*
       return SYN_OK;
     }
   } else {
-  stem_conv3x3s2_kernel<<<batch * 60, kStemThreads, 0, st>>>(x, h->dconv[0].w, h->dconv[0].bias,
-                                                            h->buf_io[cur], batch);
+  stem_conv3x3s2_kernel<true><<<batch * 60, kStemThreads, 0, st>>>(x, h->dconv[0].w, h->dconv[0].bias,
+                                                                  h->buf_io[cur], batch, nullptr);
   SYN_LAUNCH_CHECK("stem_conv3x3s2_kernel");
   mark(h, st, "stem_conv3x3s2_kernel");
   if (stop_layer == 0) return dbg(0, h->buf_io[cur]);
@@ -744,6 +749,7 @@ void syn_destroy(syn_handle_t* h) {
   cudaDeviceSynchronize();
   syn_heads_destroy(h->heads);
   syn_resnet_destroy(h->resnet);
+  syn_resnest_destroy(h->resnest);
   cudaFree(h->d_weights); cudaFree(h->d_head_w); cudaFree(h->d_head_b); cudaFree(h->d_mean);
   cudaFree(h->d_std); cudaFree(h->d_sparse); cudaFree(h->d_dense); cudaFree(h->d_tcw); cudaFreeHost(h->d_err); cudaFree(h->d_sat); cudaFree(h->d_fused); cudaFree(h->d_tc_oscale);
   cudaFree(h->buf_io[0]); cudaFree(h->buf_io[1]); cudaFree(h->buf_hid); cudaFree(h->buf_dw);
@@ -1337,3 +1343,4 @@ int syn_debug_forward_until(syn_handle_t* h, const float* x, int batch, int laye
 
 #include "heads_host.inl"
 #include "resnet_host.inl"
+#include "resnest_host.inl"

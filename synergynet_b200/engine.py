@@ -409,6 +409,39 @@ class Engine:
             self._done()
         return out, pool
 
+    # ---- ResNeSt-50 backbone variant (I2P with arch 'resnest*', model_building.py:48-49) ---------------------------------
+    def load_resnest50(self, sd: Dict[str, torch.Tensor], prefix: str = '') -> None:
+        """Hand a ``ResNeSt.resnest50()`` state dict to the library: the 87 layers in execution order (conv weight, conv
+        bias where the layer has one, its BatchNorm where it has one) and the three evaluated Linear heads concatenated
+        in the reference's output order ori | shape | exp (ResNeSt/resnet.py:316-320)."""
+        from .backbone import resnest50_layer_keys
+        bn_fields = ('weight', 'bias', 'running_mean', 'running_var')
+        with self._lock:
+            for i, (ck, bk) in enumerate(resnest50_layer_keys()):
+                w = _host_f32(sd[f'{prefix}{ck}.weight'])
+                b = sd.get(f'{prefix}{ck}.bias')
+                b = _host_f32(b) if b is not None else None
+                bn = [_host_f32(sd[f'{prefix}{bk}.{k}']) for k in bn_fields] if bk is not None else None
+                ptrs = [t.data_ptr() for t in bn] if bn is not None else [None] * 4
+                _lib.check(self._lib.syn_resnest_set_layer(self._h, i, w.data_ptr(), w.numel(),
+                                                           b.data_ptr() if b is not None else None, *ptrs, 1e-5))
+            order = ('fc_ori', 'fc_shape', 'fc_exp')
+            w = torch.cat([_host_f32(sd[f'{prefix}{k}.weight']) for k in order]).contiguous()
+            b = torch.cat([_host_f32(sd[f'{prefix}{k}.bias']) for k in order]).contiguous()
+            _lib.check(self._lib.syn_resnest_set_heads(self._h, w.data_ptr(), b.data_ptr()))
+            _lib.check(self._lib.syn_resnest_commit(self._h))
+
+    def forward_resnest50(self, x: torch.Tensor):
+        """ResNet.forward of ResNeSt-50 (ResNeSt/resnet.py:298-324): (B,3,120,120) -> ((B,62) ori|shape|exp, (B,2048) pooled)."""
+        x = self._check_x(x)
+        b = x.shape[0]
+        out = torch.empty((b, N_PARAMS), device=self.device, dtype=torch.float32)
+        pool = torch.empty((b, 2048), device=self.device, dtype=torch.float32)
+        with self._lock:
+            _lib.check(self._lib.syn_resnest50_forward(self._h, x.data_ptr(), b, out.data_ptr(), pool.data_ptr(), self._stream()))
+            self._done()
+        return out, pool
+
     def debug_forward_until(self, x: torch.Tensor, layer: int) -> torch.Tensor:
         x = self._check_x(x)
         spec = conv_plan()[layer]

@@ -102,12 +102,18 @@ class I2P(nn.Module):
             # fact 4).  Adapter used here (and by the oracle / golden vectors): params = out[:, :62] (ori|shape|exp),
             # avgpool = the 2048-d pooled feature.
             self.backbone = mobilenetv2_backbone.resnet50(pretrained=False)
-        elif any(k in self.args.arch for k in ('mobilenet', 'resnet', 'ghostnet', 'resnest')):
-            raise RuntimeError(f"arch '{args.arch}': mobilenet_v2 and resnet50 are built for sm_100a "
+        elif 'resnest' in self.args.arch:
+            # the reference builds resnest50() for ANY arch containing 'resnest' (model_building.py:48-49); it returns
+            # (params62, avgpool2048) exactly as I2P unpacks (ResNeSt/resnet.py:298-324), so no adapter is needed.
+            self.backbone = mobilenetv2_backbone.resnest50(pretrained=False)
+        elif any(k in self.args.arch for k in ('mobilenet', 'resnet', 'ghostnet')):
+            raise RuntimeError(f"arch '{args.arch}': mobilenet_v2, resnet50 and resnest50 are built for sm_100a "
                                '(SURVEY.md section 8; the other backbones are not on the hot path)')
         else:
             raise RuntimeError("Please choose [mobilenet_v2, mobilenet_1, resnet50, or ghostnet]")
-        self._is_resnet = self.args.arch == 'resnet50'
+        # the variant backbones run on their own library entry points (None: MobileNetV2, the fused default path)
+        self._variant = 'resnet50' if self.args.arch == 'resnet50' else 'resnest50' if 'resnest' in self.args.arch else None
+        self._is_resnet = self._variant is not None
         object.__setattr__(self, '_rt', _Runtime())
         object.__setattr__(self, '_basis_provider', None)
 
@@ -121,8 +127,9 @@ class I2P(nn.Module):
         return self._rt.get(device, self._backbone_sd, self._basis_provider)
 
     def _resnet_engine(self, device) -> Engine:
-        """Engine with the ResNet-50 weights: the shared library state (error flag, 3DMM bases for reconstruct) comes from
-        a commit of the MobileNetV2 path with a zero checkpoint of the right schema, then the ResNet layers are handed over."""
+        """Engine with the weights of the variant backbone (ResNet-50 or ResNeSt-50): the shared library state (error flag,
+        3DMM bases for reconstruct) comes from a commit of the MobileNetV2 path with a zero checkpoint of the right schema,
+        then the variant's layers are handed over."""
         rt = self._rt
         if not hasattr(rt, '_mbv2_stub'):
             rt._mbv2_stub = {k: v for k, v in mobilenetv2_backbone.mobilenet_v2().state_dict().items()
@@ -130,12 +137,13 @@ class I2P(nn.Module):
         eng = rt.get(device, lambda: rt._mbv2_stub, self._basis_provider)
         sd = self._backbone_sd()
         sig = rt._signature(list(sd.values()))
-        key = (eng.device.index, 'resnet50')
+        key = (eng.device.index, self._variant)
+        attr = f'_{self._variant}_commit_of'
         with rt._lock:
-            if rt._pn_sig.get(key) != sig or getattr(eng, '_resnet_commit_of', None) is not rt._sig.get(eng.device.index):
-                eng.load_resnet50(sd)
+            if rt._pn_sig.get(key) != sig or getattr(eng, attr, None) is not rt._sig.get(eng.device.index):
+                getattr(eng, f'load_{self._variant}')(sd)
                 rt._pn_sig[key] = sig
-                eng._resnet_commit_of = rt._sig.get(eng.device.index)
+                setattr(eng, attr, rt._sig.get(eng.device.index))
         return eng
 
     def _compute_device(self, t: Optional[torch.Tensor] = None) -> torch.device:
@@ -154,9 +162,11 @@ class I2P(nn.Module):
         """Testing time forward -> (param62, avgpool1280) (model_building.py:59-62).  A CPU input is moved to the
         compute GPU and the results come back on the CPU, as the reference's CPU model would return them."""
         dev = self._compute_device(input)
-        if self._is_resnet:
+        if self._variant == 'resnet50':
             out, pool = self._engine(dev).forward_resnet50(input.to(dev))
             params = out[:, :62].contiguous()
+        elif self._variant == 'resnest50':
+            params, pool = self._engine(dev).forward_resnest50(input.to(dev))
         else:
             params, pool = self._engine(dev).forward(input.to(dev), want_pool=True)
         if not input.is_cuda:
@@ -271,9 +281,9 @@ class _SynergyBase(nn.Module):
         _3D_attr, avgpool = self.I2P.forward_test(input.to(dev))
         if avgpool.shape[1] != 1280:
             raise RuntimeError('SynergyNet.forward: MLP_for.conv6 is hard-wired to a 1280-d image feature '
-                               '(pointnet_backbone.py:15,58: 2418 = 64 + 1024 + 1280 + 40 + 10); the resnet50 backbone pools '
-                               f'{avgpool.shape[1]} channels, so the refinement head cannot follow it (the reference fails '
-                               'here too, SURVEY.md fact 4).  Use forward_test() / reconstruct_vertex_62() with resnet50.')
+                               f'(pointnet_backbone.py:15,58: 2418 = 64 + 1024 + 1280 + 40 + 10); the {self.I2P.args.arch} backbone '
+                               f'pools {avgpool.shape[1]} channels, so the refinement head cannot follow it (the reference fails '
+                               f'here too, SURVEY.md fact 4).  Use forward_test() / reconstruct_vertex_62() with {self.I2P.args.arch}.')
         _3D_attr_GT = target.to(device=dev, dtype=torch.float32)
         vertex_lmk = eng.reconstruct(_3D_attr, dense=False)
         vertex_GT_lmk = eng.reconstruct(_3D_attr_GT, dense=False)
